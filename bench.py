@@ -1,6 +1,7 @@
 """Benchmark of the PonderV2 pretraining hot path on B200 (BASELINE.json metric).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload c2|c3|c4|c1]
+                    [--dump-outputs DIR]
 
 One "step" = one full pretraining iteration on one synthetic scene per GPU: SpUNet backbone forward/backward (rulebooks
 rebuilt every step), densify, dense projection, NeuS render of R rays x S samples with its second-order backward,
@@ -24,6 +25,12 @@ c3 = configs[2] (200 k voxels, 8192 rays, bf16 autocast backbone), c4 = configs[
 `--impl reference` times the reference's own algorithm on the CPU (oracle port: spconv is not installable offline and
 smooth_sampler is CUDA-only, see DESIGN.md) with every host thread; each step is a bounded sample of the workload sized
 from a calibration step so that the whole run stays within a few minutes.
+
+`--dump-outputs DIR` writes what the last step of the device-resident loop computed (see `dump_outputs`) as
+DIR/<name>.npy.  Scene, model and jitter are seeded, so two builds run with the same arguments can be compared output
+for output.  The outputs are not bitwise reproducible: the sparse convolutions reduce with fp32 atomics, and every
+training step amplifies the reordering.  Two runs of one build with --steps 20 --warmup 3 (B200, 1000 W power limit)
+differed by 3e-3 relative in the loss and by 3e-3 relative L2 in param_sample, so compare with a tolerance above that.
 """
 from __future__ import annotations
 
@@ -369,6 +376,20 @@ def build_model(wl: dict, dev, overlap: bool = True):
     return model, flat, opt
 
 
+def dump_outputs(path: str, out: dict, flat, sample: int = 1 << 22) -> None:
+    """What a caller of the training step receives from its last run, as float32 .npy files under `path`: every entry of
+    the step's output dict (the loss and its terms) and the parameters after the optimizer step.  The flat parameter
+    buffer holds ~40 M values, so `param_sample` is the value at `sample` positions drawn with a fixed seed (16 MB)."""
+    d = Path(path)
+    d.mkdir(parents=True, exist_ok=True)
+    for k, v in out.items():
+        np.save(d / f"{k}.npy", v.float().cpu().numpy())
+    n = flat.flat_param.numel()
+    idx = np.sort(np.random.default_rng(0).choice(n, size=min(n, sample), replace=False))
+    idx = torch.from_numpy(idx).to(flat.flat_param.device)
+    np.save(d / "param_sample.npy", flat.flat_param[idx].float().cpu().numpy())
+
+
 def nccl_summary(path_glob: str) -> dict:
     """Algorithm / protocol / transport lines NCCL logged for the all-reduce (NCCL_DEBUG=INFO to per-rank files)."""
     import glob
@@ -441,7 +462,7 @@ def run_ours(args, wl: dict) -> None:
     shape = (torch.from_numpy(scene["grid_coord"]).max(0).values + 96).tolist()
     loss_host = torch.zeros(1).pin_memory()
 
-    def step(inputs: dict) -> torch.Tensor:
+    def step(inputs: dict) -> dict:
         data = dict(inputs)
         data["sparse_shape"] = shape
         opt.zero_grad()                     # the flat gradient buffer is zeroed, views stay attached
@@ -450,7 +471,7 @@ def run_ours(args, wl: dict) -> None:
         out["loss"].backward()              # gradient slices are all-reduced from hooks while this runs (N > 1)
         flat.all_reduce_mean()
         opt.step()
-        return out["loss"].detach()
+        return {k: v.detach() for k, v in out.items()}
 
     def barrier():
         if world > 1:
@@ -478,10 +499,10 @@ def run_ours(args, wl: dict) -> None:
         for _ in range(args.steps):
             if from_host:
                 inputs = {k: v.to(dev, non_blocking=True) for k, v in host.items()}
-                loss = step(inputs)
-                loss_host.copy_(loss.reshape(1), non_blocking=True)
+                out = step(inputs)
+                loss_host.copy_(out["loss"].reshape(1), non_blocking=True)
             else:
-                loss = step(resident)
+                out = step(resident)
         e1.record()
         barrier()
         gc.enable()
@@ -490,7 +511,7 @@ def run_ours(args, wl: dict) -> None:
         t = torch.tensor([ms], device=dev)
         if world > 1:
             dist.all_reduce(t, op=dist.ReduceOp.MAX)
-        return t.item(), lib.pv2_launch_count() - l0, float(loss)
+        return t.item(), lib.pv2_launch_count() - l0, out
 
     log(f"model + scene ready on rank {rank}/{world}: {wl['voxels']} voxels, {wl['rays']} rays")
     # The clock sampler is started BEFORE the warm-up: nvidia-smi's start-up (fork + NVML attaching to the device)
@@ -512,8 +533,13 @@ def run_ours(args, wl: dict) -> None:
         return
     if rank == 0:
         clocks.wait_first_sample()
-    ms_dev, launches, last_loss = timed_loop(from_host=False, profile=False)      # `value`: un-instrumented
+    ms_dev, launches, last_out = timed_loop(from_host=False, profile=False)       # `value`: un-instrumented
     log(f"device-resident loop: {ms_dev / args.steps:.2f} ms/step")
+    last_loss = float(last_out["loss"])
+    if args.dump_outputs and rank == 0:
+        # before the two loops below move the parameters on
+        dump_outputs(args.dump_outputs, last_out, flat)
+        log(f"outputs of the last device-resident step written to {args.dump_outputs}")
     ms_e2e, _, _ = timed_loop(from_host=True, profile=False)
     log(f"host-fed loop: {ms_e2e / args.steps:.2f} ms/step")
     clk = clocks.stop() if rank == 0 else None
@@ -597,7 +623,13 @@ def main() -> None:
                          "all-reduces overlapped with it (A/B switch)")
     ap.add_argument("--profile-step", action="store_true",
                     help="run one warmed-up step inside cudaProfilerStart/Stop and exit (for ncu --profile-from-start off)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the outputs of the last timed device-resident step to DIR/<name>.npy (float32)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl == "reference" or args.profile_step):
+        ap.error("--dump-outputs needs the timed loops of --impl ours (not --profile-step)")
     wl = dict(WORKLOADS[args.workload])
     if args.projection == "unet3d":
         if wl["outdoor"] or args.impl == "reference":
